@@ -7,6 +7,7 @@ step so that one step's inputs (Q x 64 MB) exceed the 126 MB L2.  Metric: input 
 second, bit-exact vs the CPU oracle (every query of the step is checked).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c2dense]
+                  [--dump-outputs DIR]
 
 value   device-resident: lists already in HBM, one batched launch per step, CUDA events on the launching stream.
 e2e     the same step through the host-pointer C ABI, HOST buffers, copies inside the timed region.  The
@@ -24,6 +25,12 @@ overlaps the filter of step i+1.
 `--impl reference` times the reference's CPU algorithm (the C oracle restating algo/uidlist.go; the Go
 toolchain is absent) on the same workload -- N x Q queries at N GPUs -- one query per host thread, the only
 parallelism the reference has for this path (IntersectSorted itself is single-threaded).
+
+`--dump-outputs DIR` writes the result of the last timed step of the device-resident loop, as a caller of
+dgx_dev_filter_batch receives it, to DIR/offsets.npy (Q + 1 per-query offsets) and DIR/uids.npy (the
+concatenated result UIDs), both float64.  The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.  At N > 1 every rank writes its own queries' result, named
+offsets_rank<r>.npy and uids_rank<r>.npy.
 """
 from __future__ import annotations
 
@@ -124,6 +131,26 @@ def cpu_intersect_batch(orc, queries, threads: int) -> float:
         with ThreadPoolExecutor(max_workers=threads) as ex:  # ctypes releases the GIL
             list(ex.map(orc.intersect_sorted, queries))
     return time.perf_counter() - t0
+
+
+DUMP_MAX_BYTES = 64 << 20  # --dump-outputs budget over all ranks' files
+
+
+def dump_outputs(out_dir: str, offsets: np.ndarray, uids: np.ndarray, rank: int, world: int):
+    """Writes one step's result as float64 .npy files.  float64 holds every UID below 2^53 exactly, which
+    covers these workloads (masters of <= 4e6 gaps of <= 2^20).  A result larger than this rank's share of
+    DUMP_MAX_BYTES is replaced by a fixed, seeded sample of its positions, written as uids_index.npy."""
+    if uids.size and int(uids.max()) >= 1 << 53:
+        raise SystemExit("--dump-outputs: a result UID does not fit float64 exactly")
+    arrays = {"offsets": offsets, "uids": uids}
+    room = DUMP_MAX_BYTES // world - 8 * offsets.size
+    if 8 * uids.size > room:
+        idx = np.sort(np.random.default_rng(0).choice(uids.size, room // 16, replace=False))
+        arrays["uids"], arrays["uids_index"] = uids[idx], idx
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a.astype(np.float64))
 
 
 def workload_config(q: int, world: int, workload: str = "c2"):
@@ -353,7 +380,10 @@ def main():
     ap.add_argument("--no-dense", action="store_true", help="skip the p=0.9 variant of the headline step")
     ap.add_argument("--no-resident", action="store_true", help="do not declare the lists resident (no pre-pass / pipeline overlap across steps)")
     ap.add_argument("--no-e2e", action="store_true", help="kernel iteration runs only: skip the end-to-end legs (the line then has no e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result to DIR/*.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -508,6 +538,9 @@ def main():
         dist.barrier()
     clocks = sampler.stop()
     launches = int(lib.dgx_lane_launches(lane) - launches0)
+    if args.dump_outputs:
+        last = bufs[(args.steps - 1) % NBUF].cpu().numpy().view(np.uint64)
+        dump_outputs(args.dump_outputs, last[: Q + 1], last[Q + 1: Q + 1 + int(last[Q])], rank, world)
     total_ms = evs[0].elapsed_time(ev_end)
     step_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     bit_exact = bit_exact and rc_sync == 0

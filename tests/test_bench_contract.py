@@ -1,10 +1,12 @@
-"""bench.py's driver-facing contract that can be checked without a GPU: the reference arm prints one JSON
-line with the agreed keys, and the product arm refuses to run without CUDA (no CPU fallback)."""
+"""bench.py's command-line contract: the reference arm prints one JSON line with the agreed keys, the product
+arm refuses to run without CUDA (no CPU fallback), and --dump-outputs writes the timed step's result (checked
+against the oracle on a GPU)."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -56,6 +58,59 @@ def test_reference_arm_other_ranks_exit_quietly():
     r = run("--impl", "reference", "--gpus", "2", "--queries", "2", "--steps", "1", "--warmup", "0",
             env={"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"})
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_files_and_budget(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+
+    offsets = np.array([0, 3, 5], np.uint64)
+    uids = np.array([1, 7, 9, 2, (1 << 53) - 1], np.uint64)
+    bench.dump_outputs(str(tmp_path / "a"), offsets, uids, 0, 1)
+    assert sorted(os.listdir(tmp_path / "a")) == ["offsets.npy", "uids.npy"]
+    got = np.load(tmp_path / "a" / "uids.npy")
+    assert got.dtype == np.float64 and np.array_equal(got.astype(np.uint64), uids)
+    assert np.array_equal(np.load(tmp_path / "a" / "offsets.npy"), offsets.astype(np.float64))
+
+    # over budget: a seeded sample of positions, the same from run to run, within the byte budget
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 2 * (8 * 3 + 16 * 100))
+    big = np.arange(10_000, dtype=np.uint64) * 3
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), offsets, big, 1, 2)
+    names = ["offsets_rank1.npy", "uids_index_rank1.npy", "uids_rank1.npy"]
+    assert sorted(os.listdir(tmp_path / "b")) == names
+    assert sum(os.path.getsize(tmp_path / "b" / n) - 128 for n in names) <= bench.DUMP_MAX_BYTES // 2
+    idx = np.load(tmp_path / "b" / "uids_index_rank1.npy").astype(np.int64)
+    assert idx.size == 100 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(np.load(tmp_path / "b" / "uids_rank1.npy"), big[idx].astype(np.float64))
+    for n in names:
+        assert np.array_equal(np.load(tmp_path / "b" / n), np.load(tmp_path / "c" / n))
+
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "d"), offsets, np.array([1 << 53], np.uint64), 0, 1)
+
+
+def test_steps_must_be_positive():
+    r = run("--steps", "0")
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_timed_result(tmp_path, orc):
+    """The dumped arrays are the last timed step's per-query results, equal to the oracle on the seeded inputs."""
+    r = run("--steps", "3", "--warmup", "0", "--queries", "2", "--no-e2e", "--no-ops", "--no-dense",
+            "--dump-outputs", str(tmp_path))
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout.strip().splitlines()[-1])
+    assert d["steps"] == 3 and d["bit_exact"] is True
+    sys.path.insert(0, ROOT)
+    import bench
+
+    off = np.load(tmp_path / "offsets.npy").astype(np.int64)
+    uids = np.load(tmp_path / "uids.npy").astype(np.uint64)
+    assert off.size == 3 and off[-1] == uids.size == d["out_uids_per_step"]
+    for i, q in enumerate(bench.make_queries(2, 0)):
+        assert np.array_equal(uids[off[i]:off[i + 1]], orc.intersect_sorted(q))
 
 
 def test_product_arm_needs_cuda():

@@ -35,8 +35,6 @@ struct DPack {
     const unsigned char* deltas;  // 16-byte aligned, >= 32 bytes of slack after the end
     const u64* uid_off;    // nblocks + 1: exclusive prefix of num
     u32 max_num;           // largest NumUids of any block
-    u32 sysmem;            // base / num / delta_off / deltas are mapped pinned HOST memory (zero-copy decode):
-                           // the window is filled with plain vector loads over PCIe instead of a TMA bulk copy
 };
 struct DSeek {            // written by decode_seek_kernel
     u64 first_block;
@@ -121,10 +119,6 @@ __device__ __forceinline__ void mbar_wait(u32 bar, u32 parity) {
 // backs off with nanosleep, so a waiting warp does not compete with working warps for issue slots.
 template <unsigned kSleepNs = 128>
 __device__ __forceinline__ void mbar_wait_relaxed(u32 bar, u32 parity) {
-#ifdef DGX_HWWAIT
-    mbar_wait(bar, parity);   // experiment: leave the waiting to the hardware's try_wait suspension
-    return;
-#endif
     u32 done = 0;
     while (true) {
         asm volatile(
@@ -211,28 +205,13 @@ __device__ __forceinline__ void decode_warp_run(const DPack& pk, u64 first_block
 
         // ---- (1) TMA bulk copy of the batch's delta bytes ------------------------
         const u32 bytes = (u32)(((wend - win0) + 15ull) & ~15ull);
-        if (pk.sysmem) {
-            // Zero-copy: the pack's bytes are read straight from pinned host memory by the lanes (16 bytes each,
-            // all requests of the window in flight together); thousands of resident warps keep PCIe full without
-            // the per-copy set-up a DMA of every small pack costs, and nothing compressed is staged in HBM.
-            const uint4* src = reinterpret_cast<const uint4*>(pk.deltas + win0);
-            uint4* dstw = reinterpret_cast<uint4*>(S.payload);
-            for (u32 o = lane; o < bytes / 16u; o += 32) {
-                uint4 q;
-                asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];"
-                             : "=r"(q.x), "=r"(q.y), "=r"(q.z), "=r"(q.w) : "l"(src + o));
-                dstw[o] = q;
-            }
-            __syncwarp();
-        } else {
-            if (lane == 0) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                mbar_expect_tx(bar, bytes);
-                tma_bulk_g2s(smem_u32(S.payload), pk.deltas + win0, bytes, bar);
-            }
-            mbar_wait(bar, parity);
-            parity ^= 1u;
+        if (lane == 0) {
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            mbar_expect_tx(bar, bytes);
+            tma_bulk_g2s(smem_u32(S.payload), pk.deltas + win0, bytes, bar);
         }
+        mbar_wait(bar, parity);
+        parity ^= 1u;
 
         // ---- (2) tag walk: lane i records the byte offset of every group of block i
         if (lane < nb) {

@@ -76,23 +76,13 @@ static std::vector<dgx_lane*> g_pool;  // idle lanes for the host-pointer entry 
 static std::condition_variable g_pool_cv;
 static size_t g_lanes_out = 0;     // lanes currently leased
 static size_t g_lanes_total = 0;   // lanes in existence (pooled + leased)
-static u32 g_stream_ratio = 16;
-static u32 g_scap_override = 0;       // DGX_SCAP: force the filter kernel's slice staging capacity
+constexpr u32 kStreamRatio = 16;       // filter_kernel: stream an oversized slice when it is <= 16 x the live candidates
 constexpr u32 kScapMin = 8192, kScapMax = 65536;  // bytes
 static int g_filter_pipe = 1;          // DGX_FILTER=v4 selects the non-persistent kernel
 static int g_merge_multi = 1;          // DGX_MERGE=tree forces the pairwise merge tree
-static int g_merge_lag = 0;            // DGX_MERGE_LAG: a merge CTA moves the tile this many tiles back to the output; 0 = scan + compact kernels
-                                       // (default: measured faster, 1.655 vs 1.69 ms at 888 on C5 -- the copy is not hidden under the merging)
 static int g_merge_ahead = -1;         // DGX_MERGE_AHEAD: L2 prefetch distance in tiles (-1 = 3 x SM count, the resident CTAs; 0 = off)
-static int g_merge_t32 = 1;            // DGX_MERGE=levels: the round-1 pipeline (64-bit levels engine, boundary-major bounds)
-static u32 g_merge_stride = 0;         // DGX_MERGE_STRIDE: sample gaps per multiway-merge tile (tile ~ 512 x stride values); 0 = 10 for the
-                                       // 32-bit engine (7680-slot rounds), 6 for DGX_MERGE=levels (4096-slot rounds)
-static int g_zero_copy = 0;            // DGX_ZERO_COPY=1: decode pinned packs in place over PCIe (measured slower than DMA: 35 vs 43 GB/s)
-static size_t g_merge_multi_min = size_t(1) << 18;  // totals below this stay on the tree (fewer launches)
-static size_t g_pre_throttle_smem = 0;  // DGX_PRE_THROTTLE: dynamic smem asked for by an ahead-of-time pre-pass (0 = unthrottled)
-static u32 g_reserve_ctas = 0;         // DGX_RESERVE_CTAS: pipeline CTAs left out of the persistent grid
-static uint64_t g_pipe_min_values = 0;  // DGX_PIPE_MIN_VALUES: batches driving fewer values than this use filter_kernel
-static size_t g_pipe_min_k = 2;        // DGX_PIPE_MIN_K: batches whose widest query has fewer lists use filter_kernel
+static u32 g_merge_stride = 10;        // DGX_MERGE_STRIDE: sample gaps per multiway-merge tile (tile ~ 512 x stride values, 7680-slot rounds)
+static size_t g_merge_multi_min = size_t(1) << 18;  // DGX_MERGE_MULTI_MIN: totals below this stay on the tree (fewer launches)
 static int g_num_sms = 148;
 constexpr size_t kPipeSmemMax = 220 * 1024;
 
@@ -241,6 +231,14 @@ static int lane_begin_op(dgx_lane* l) {
     return DGX_OK;
 }
 
+// Call after every kernel launch on the lane's stream: reports a failed launch and counts the launch.
+static int launched(dgx_lane* l) {
+    CK(cudaGetLastError());
+    l->launches += 1;
+    g_stats.launches += 1;
+    return DGX_OK;
+}
+
 // ---------------------------------------------------------------------------
 // lifecycle
 // ---------------------------------------------------------------------------
@@ -270,15 +268,13 @@ extern "C" int dgx_init(int device) {
                             (int)(2 * F_TA * sizeof(u64) + kScapMax)));
     CK(cudaFuncSetAttribute(filter_pipe_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPipeSmemMax));
     CK(cudaFuncSetAttribute(filter_pipe_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPipeSmemMax));
-    CK(cudaFuncSetAttribute(mmerge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * MM_CP * sizeof(u64))));
     g_num_sms = prop.multiProcessorCount;
     numa_probe(device);
     if (const char* s = getenv("DGX_FILTER")) g_filter_pipe = (strcmp(s, "v4") != 0);
     CK(cudaFuncSetAttribute(mmerge3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T_SMEM));
-    if (const char* s = getenv("DGX_MERGE")) { g_merge_multi = (strcmp(s, "tree") != 0); g_merge_t32 = (strcmp(s, "levels") != 0); }
-    if (const char* s = getenv("DGX_ZERO_COPY")) g_zero_copy = atoi(s) != 0;
+    if (const char* s = getenv("DGX_MERGE")) g_merge_multi = (strcmp(s, "tree") != 0);
+    if (const char* s = getenv("DGX_MERGE_MULTI_MIN")) g_merge_multi_min = (size_t)atoll(s);
     if (const char* s = getenv("DGX_MERGE_AHEAD")) g_merge_ahead = atoi(s);
-    if (const char* s = getenv("DGX_MERGE_LAG")) g_merge_lag = atoi(s);
     if (const char* s = getenv("DGX_MERGE_STRIDE")) { const int v = atoi(s); if (v >= 1 && v <= 16) g_merge_stride = (u32)v; }
     g_device = device;
     return DGX_OK;
@@ -508,16 +504,8 @@ static int filter_batch_impl(dgx_lane* l, int op, const ListDesc* lists, const s
     uint64_t ntiles = 0, uids_in = 0;
     size_t li = 0, kmax = 1;
     for (size_t q = 0; q < nq; ++q) kmax = std::max(kmax, k_off[q + 1] - k_off[q]);
-    // Small batches take the single-launch kernel: the pipeline's plan pre-pass (two more launches, a second
-    // descriptor copy) costs more than it saves when the whole batch is a few hundred tiles (DGX_PIPE_MIN_VALUES).
-    uint64_t drive_total = 0;
-    for (size_t q = 0; q < nq; ++q) {
-        uint64_t mn = UINT64_MAX;
-        for (size_t i = k_off[q]; i < k_off[q + 1]; ++i) mn = std::min<uint64_t>(mn, lists[i].len);
-        if (op == DGX_OP_DIFFERENCE && k_off[q + 1] > k_off[q]) mn = lists[k_off[q]].len;
-        if (mn != UINT64_MAX) drive_total += mn;
-    }
-    const bool use_pipe = g_filter_pipe && kmax >= g_pipe_min_k && drive_total >= g_pipe_min_values;
+    // batches of single-list queries take filter_kernel
+    const bool use_pipe = g_filter_pipe && kmax >= 2;
     // 2-list batches: 1024-value tiles (per-tile overheads over twice the values); wider queries: 512 (filter_pipe.cuh)
     const int pipe_va = kmax <= 2 ? 4 : 2;
     const uint64_t tile_sz = use_pipe ? (uint64_t)p_tile_size(pipe_va) : (uint64_t)F_TA;
@@ -581,10 +569,9 @@ static int filter_batch_impl(dgx_lane* l, int op, const ListDesc* lists, const s
     P.ntasks = (u32)nq;
     P.ntiles = (u32)ntiles;
     P.op = op;
-    P.stream_ratio = g_stream_ratio;
+    P.stream_ratio = kStreamRatio;
     // staging capacity (bytes): ~1.1 tile-widths of 32-bit keys for every filter list of the widest query
-    P.scap_bytes = g_scap_override ? g_scap_override
-                                   : (u32)std::min<size_t>(32768, std::max<size_t>(kScapMin, (kmax - 1) * 1152 * 4));
+    P.scap_bytes = (u32)std::min<size_t>(32768, std::max<size_t>(kScapMin, (kmax - 1) * 1152 * 4));
     P.out = (u64*)d_out;
     P.out_cap = out_cap;
     P.out_off = (u64*)d_out_off;
@@ -593,9 +580,7 @@ static int filter_batch_impl(dgx_lane* l, int op, const ListDesc* lists, const s
     P.err = l->d_err;
     if (!use_pipe) {
         filter_kernel<<<(unsigned)ntiles, F_NT, 2 * F_TA * sizeof(u64) + P.scap_bytes, l->stream>>>(P);
-        CK(cudaGetLastError());
-        l->launches += 1;
-        g_stats.launches += 1;
+        if (int e = launched(l)) return e;
     } else {
         // ---- persistent TMA pipeline: plan pre-pass + filter_pipe_kernel ----------------
         void* hp_raw;
@@ -616,23 +601,15 @@ static int filter_batch_impl(dgx_lane* l, int op, const ListDesc* lists, const s
         rc = ar->alloc((npairs + 1) * sizeof(PPlanEntry), &d_plan);
         if (rc) return rc;
         CK(cudaMemcpyAsync(d_pb, h_pb, nq * sizeof(u64), cudaMemcpyHostToDevice, pre));
-        // DGX_PRE_THROTTLE: dynamic shared memory an ahead-of-time pre-pass asks for (16 KB would limit it to one CTA on
-        // an SM that holds two pipeline CTAs).  Measured: no effect (0.3559 vs 0.3565 ms) -- what the overlap costs the
-        // pipeline is L2 / DRAM interference, not issue slots -- so the default is 0.
-        const size_t pre_smem = ahead ? g_pre_throttle_smem : 0;
-        filter_tiles_kernel<<<(unsigned)((ntiles + 255) / 256), 256, pre_smem, pre>>>(P.tasks, P.lists, (const u64*)d_pb, P.ntasks,
-                                                                                      P.ntiles, (PTileEntry*)d_tiles, (u32)tile_sz);
-        CK(cudaGetLastError());
-        l->launches += 1;
-        g_stats.launches += 1;
+        filter_tiles_kernel<<<(unsigned)((ntiles + 255) / 256), 256, 0, pre>>>(P.tasks, P.lists, (const u64*)d_pb, P.ntasks,
+                                                                               P.ntiles, (PTileEntry*)d_tiles, (u32)tile_sz);
+        if (int e = launched(l)) return e;
         if (npairs) {
             const u64 blocks = (npairs + 255) / 256;
             if (blocks > 0x7fffffffull) return fail(DGX_ERR_ARG, "batch too large");
-            filter_plan_kernel<<<(unsigned)blocks, 256, pre_smem, pre>>>(P.tasks, P.lists, (const u64*)d_pb, P.ntasks, npairs,
-                                                                         (PPlanEntry*)d_plan, (u32)tile_sz);
-            CK(cudaGetLastError());
-            l->launches += 1;
-            g_stats.launches += 1;
+            filter_plan_kernel<<<(unsigned)blocks, 256, 0, pre>>>(P.tasks, P.lists, (const u64*)d_pb, P.ntasks, npairs,
+                                                                  (PPlanEntry*)d_plan, (u32)tile_sz);
+            if (int e = launched(l)) return e;
         }
         PParams PP;
         PP.f = P;
@@ -647,7 +624,6 @@ static int filter_batch_impl(dgx_lane* l, int op, const ListDesc* lists, const s
         // staged slices: ~1.125 tile-widths per filter list; a 2-list batch stages up to 2.25 tile-widths of its one
         // filter list (size ratios beyond that probe the list in HBM, the reference's own Jump / Bin regimes)
         size_t cap = (TA + TA / 8) * nl * (kmax <= 2 ? 2 : 1);
-        if (g_scap_override) cap = g_scap_override / 8;
         cap = std::min<size_t>(std::max<size_t>(cap, TA + TA / 8), 9216) & ~size_t(1);
         PP.slice_cap = (u32)cap;
         const size_t smem = ((sizeof(PShared) + 127) & ~size_t(127)) + (1 + P_OS) * TA * sizeof(u64) +
@@ -657,19 +633,13 @@ static int filter_batch_impl(dgx_lane* l, int op, const ListDesc* lists, const s
         int per_sm = 0;
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, P_NT, smem));
         if (per_sm < 1) return fail(DGX_ERR_CUDA, "filter_pipe_kernel does not fit on an SM");
-        u64 resident = (u64)per_sm * (u64)g_num_sms;
-        // DGX_RESERVE_CTAS: leave a few CTA slots free so that a collective queued on another stream (the result
-        // gather of the previous batch) finds an SM while the persistent pipeline runs
-        if (g_reserve_ctas && resident > 2 * (u64)g_reserve_ctas) resident -= g_reserve_ctas;
-        PP.nctas = (u32)std::min<u64>(resident, ntiles);
+        PP.nctas = (u32)std::min<u64>((u64)per_sm * (u64)g_num_sms, ntiles);
         if (ahead) {
             CK(cudaEventRecord(l->ev_plan[slot], l->side));
             CK(cudaStreamWaitEvent(l->stream, l->ev_plan[slot], 0));
         }
         kern<<<PP.nctas, P_NT, smem, l->stream>>>(PP);
-        CK(cudaGetLastError());
-        l->launches += 1;
-        g_stats.launches += 1;
+        if (int e = launched(l)) return e;
         if (ahead) CK(cudaEventRecord(l->ev_pipe[slot], l->stream));
     }
     g_stats.uids_in += uids_in;
@@ -848,9 +818,7 @@ static int merge_tree_impl(dgx_lane* l, std::vector<MRef> cur, std::vector<uint6
         P.ticket = (u32*)(d_status + spos + L.ntiles);
         P.err = l->d_err;
         merge_kernel<<<(unsigned)L.ntiles, M_NT, 0, l->stream>>>(P);
-        CK(cudaGetLastError());
-        l->launches += 1;
-        g_stats.launches += 1;
+        if (int e = launched(l)) return e;
         tpos += L.tasks.size();
         spos += L.ntiles + 2;
     }
@@ -858,14 +826,14 @@ static int merge_tree_impl(dgx_lane* l, std::vector<MRef> cur, std::vector<uint6
     return DGX_OK;
 }
 
-// Single-pass multiway merge (merge_multi.cuh) for 3..64 runs.
+// Single-pass multiway merge (merge_multi.cuh, merge_tile32.cuh) for 3..64 runs.
 static int merge_multi_impl(dgx_lane* l, const std::vector<MRef>& runs, const std::vector<uint64_t>& ub, uint64_t total,
                             uint64_t* d_out, size_t out_cap, uint64_t* d_out_len) {
     const size_t k = runs.size();
-    // Samples per run proportional to its length.  Every 4th distinct sample becomes a splitter, so a
-    // tile is the sum of 4 sample gaps (~2K values on average, Gamma-distributed instead of
-    // exponential) and rarely overflows the 4096-value shared-memory chunk.
-    const u32 stride = g_merge_stride ? (g_merge_t32 ? g_merge_stride : std::min<u32>(g_merge_stride, 7)) : (g_merge_t32 ? 10u : 6u);
+    // About one sample per 512 values, spread over the runs in proportion to their lengths.  Every stride-th distinct
+    // sample becomes a splitter, so a tile is the sum of `stride` sample gaps (~5K values at the default 10,
+    // Gamma-distributed instead of exponential) and rarely needs more than one 7680-slot round of mmerge3_kernel.
+    const u32 stride = g_merge_stride;
     const uint64_t ntarget = std::min<uint64_t>(std::max<uint64_t>(total / 512, 1), uint64_t(1) << 24);
     std::vector<u32> soff(k + 1, 0);
     for (size_t j = 0; j < k; ++j) soff[j + 1] = soff[j] + (u32)((unsigned __int128)ub[j] * ntarget / total);
@@ -884,8 +852,7 @@ static int merge_multi_impl(dgx_lane* l, const std::vector<MRef>& runs, const st
     const size_t a_tout = a_tin + (size_t)(nsamp + 2) * 8;
     const size_t a_tcnt = a_tout + (size_t)(nsamp + 3) * 8;
     const size_t a_tlo = ((a_tcnt + (size_t)(nsamp + 2) * 4 + 255) & ~size_t(255));
-    const size_t a_status = a_tlo + (size_t)(nsamp + 2) * 8;
-    const size_t a_end = a_status + (size_t)(nsamp + 3) * 8 + 256;  // look-back words + ticket (merge_tile32.cuh, DGX_MERGE_LAG)
+    const size_t a_end = a_tlo + (size_t)(nsamp + 2) * 8;
     rc = l->ws.alloc(a_end, &d_raw);
     if (rc) return rc;
     void* d_scratch;
@@ -914,15 +881,10 @@ static int merge_multi_impl(dgx_lane* l, const std::vector<MRef>& runs, const st
     const u32 max_tiles = nsamp / stride + 1;
     P.nbs = max_tiles + 1;
     P.tile_lo = (u64*)(d + a_tlo);
-    P.lag = !g_merge_t32 || g_merge_lag < 0 ? 0u : (u32)g_merge_lag;
     P.ahead = g_merge_ahead < 0 ? 3u * (u32)g_num_sms : (u32)g_merge_ahead;
-    P.status = (u64*)(d + a_status);
-    P.ticket = (u32*)(d + a_status + (size_t)(nsamp + 3) * 8);
     if (nsamp) {
         msample_kernel<<<(nsamp + 255) / 256, 256, 0, l->stream>>>(P);
-        CK(cudaGetLastError());
-        l->launches += 1;
-        g_stats.launches += 1;
+        if (int e = launched(l)) return e;
         // the sample runs are sorted: the merge tree (with de-duplication) yields the distinct splitters
         std::vector<MRef> sruns;
         std::vector<uint64_t> sub;
@@ -938,38 +900,14 @@ static int merge_multi_impl(dgx_lane* l, const std::vector<MRef>& runs, const st
         CK(cudaMemsetAsync(d + a_nsplit, 0, 8, l->stream));
     }
     const uint64_t nb = (uint64_t)(max_tiles + 1) * k;
-    if (g_merge_t32) {
-        mplan2_kernel<<<(unsigned)((nb + 255) / 256), 256, 0, l->stream>>>(P);
-        CK(cudaGetLastError());
-        if (P.lag) CK(cudaMemsetAsync(d + a_status, 0, (size_t)(nsamp + 3) * 8 + 256, l->stream));
-        mmerge3_kernel<<<max_tiles, T_NT, T_SMEM, l->stream>>>(P);
-        CK(cudaGetLastError());
-        if (P.lag) {
-            mtail_kernel<<<std::min<u32>(P.lag, max_tiles), T_NT, 0, l->stream>>>(P);
-            CK(cudaGetLastError());
-            l->launches += 3;
-            g_stats.launches += 3;
-            return DGX_OK;
-        }
-        mscan_kernel<<<1, 1024, 0, l->stream>>>(P);
-        CK(cudaGetLastError());
-        mcompact_kernel<<<max_tiles, 256, 0, l->stream>>>(P);
-        CK(cudaGetLastError());
-        l->launches += 4;
-        g_stats.launches += 4;
-        return DGX_OK;
-    }
-    mplan_kernel<<<(unsigned)((nb + 255) / 256), 256, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
-    mmerge_kernel<<<max_tiles, MM_NT, 2 * MM_CP * sizeof(u64), l->stream>>>(P);
-    CK(cudaGetLastError());
+    mplan2_kernel<<<(unsigned)((nb + 255) / 256), 256, 0, l->stream>>>(P);
+    if (int e = launched(l)) return e;
+    mmerge3_kernel<<<max_tiles, T_NT, T_SMEM, l->stream>>>(P);
+    if (int e = launched(l)) return e;
     mscan_kernel<<<1, 1024, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
+    if (int e = launched(l)) return e;
     mcompact_kernel<<<max_tiles, 256, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
-    l->launches += 4;
-    g_stats.launches += 4;
-    return DGX_OK;
+    return launched(l);
 }
 
 extern "C" int dgx_dev_merge_sorted(dgx_lane* l, const uint64_t* const* d_lists, const size_t* lens, size_t k,
@@ -1015,10 +953,9 @@ static PackLayout pack_layout(const dgx_pack_view* v) {
     L.dpad = ((L.dbytes + 15) & ~size_t(15)) + 48;
     return L;
 }
-// Writes the metadata image at h (L.meta_bytes) and validates the block table.
-static int pack_fill_meta(const dgx_pack_view* v, const PackLayout& L, char* h, uint64_t* exact_len, uint32_t* max_num_out) {
-    const size_t nb = L.nb;
-    uint64_t* h_uoff = (uint64_t*)(h + L.o_uoff);
+// Validates the block table of v and writes its uid_off table (nblocks + 1 words) to h_uoff.
+static int pack_scan_blocks(const dgx_pack_view* v, uint64_t* h_uoff, uint64_t* exact_len, uint32_t* max_num_out) {
+    const size_t nb = v ? v->nblocks : 0;
     uint64_t acc = 0;
     uint32_t max_num = 0;
     for (size_t i = 0; i < nb; ++i) {
@@ -1036,6 +973,14 @@ static int pack_fill_meta(const dgx_pack_view* v, const PackLayout& L, char* h, 
                         i, (long long)(b1 - b0), num, (unsigned long long)need);
     }
     h_uoff[nb] = acc;
+    *exact_len = acc;
+    *max_num_out = max_num;
+    return DGX_OK;
+}
+// Writes the metadata image at h (L.meta_bytes) and validates the block table.
+static int pack_fill_meta(const dgx_pack_view* v, const PackLayout& L, char* h, uint64_t* exact_len, uint32_t* max_num) {
+    const size_t nb = L.nb;
+    if (int rc = pack_scan_blocks(v, (uint64_t*)(h + L.o_uoff), exact_len, max_num)) return rc;
     if (nb) {
         memcpy(h, v->base, nb * 8);
         memcpy(h + L.o_doff, v->delta_off, (nb + 1) * 8);
@@ -1043,8 +988,6 @@ static int pack_fill_meta(const dgx_pack_view* v, const PackLayout& L, char* h, 
     } else {
         memset(h + L.o_doff, 0, 8);
     }
-    *exact_len = acc;
-    *max_num_out = max_num;
     return DGX_OK;
 }
 static void pack_point(dgx_dev_pack* out, const dgx_pack_view* v, const PackLayout& L, char* d_meta, char* d_deltas,
@@ -1056,7 +999,6 @@ static void pack_point(dgx_dev_pack* out, const dgx_pack_view* v, const PackLayo
     out->pk.num = (const u32*)(d_meta + L.o_num);
     out->pk.deltas = (const unsigned char*)d_deltas;
     out->pk.max_num = max_num;
-    out->pk.sysmem = 0;
     out->bytes = L.meta_bytes + L.dpad;
     out->exact_len = exact_len;
     out->block_size = v ? v->block_size : 0;
@@ -1090,84 +1032,6 @@ static int pack_upload_impl(dgx_lane* l, const dgx_pack_view* v, void* d_mem_or_
     g_stats.h2d += L.meta_bytes + L.dbytes;
     pack_point(out, v, L, d, d + L.meta_bytes, exact, max_num);
     out->d_mem = d_mem;
-    return DGX_OK;
-}
-
-// Device-usable alias of a pinned (cudaMallocHost / cudaHostRegister'ed, mapped) host pointer, or nullptr.
-static const void* mapped_host_ptr(const void* p) {
-    if (!p) return nullptr;
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-    if (at.type != cudaMemoryTypeHost || !at.devicePointer) return nullptr;
-    return at.devicePointer;
-}
-
-// Zero-copy form of packs_upload_ws: when every array of every pack is pinned host memory the decode kernel
-// reads base / NumUids / delta_off / deltas directly over PCIe; only uid_off (computed here while the block table
-// is validated) is copied, one small transfer for the whole call.  Returns DGX_OK with *done = false when some
-// array is pageable (the caller then stages through DMA copies).
-static int packs_map_ws(dgx_lane* l, const dgx_pack_view* const* views, size_t k, dgx_dev_pack* outs, bool* done) {
-    *done = false;
-    if (!g_zero_copy) return DGX_OK;
-    struct Dev { const void *base, *num, *doff, *del; };
-    std::vector<Dev> dv(k);
-    size_t uoff_total = 0;
-    for (size_t i = 0; i < k; ++i) {
-        const dgx_pack_view* v = views[i];
-        if (!v) continue;
-        if (v->nblocks == 0) return DGX_OK;  // empty views carry no arrays: take the generic path
-        dv[i] = {mapped_host_ptr(v->base), mapped_host_ptr(v->num_uids), mapped_host_ptr(v->delta_off), mapped_host_ptr(v->deltas)};
-        if (!dv[i].base || !dv[i].num || !dv[i].doff || !dv[i].del) return DGX_OK;
-        if ((reinterpret_cast<uintptr_t>(dv[i].del) & 15u) || (reinterpret_cast<uintptr_t>(dv[i].base) & 7u) ||
-            (reinterpret_cast<uintptr_t>(dv[i].doff) & 7u) || (reinterpret_cast<uintptr_t>(dv[i].num) & 3u))
-            return DGX_OK;
-        uoff_total += (v->nblocks + 1) * sizeof(uint64_t);
-    }
-    if (uoff_total == 0) return DGX_OK;
-    void *d_raw, *h_raw;
-    int rc = l->ws.alloc(uoff_total, &d_raw);
-    if (rc) return rc;
-    rc = l->host.alloc(uoff_total, &h_raw);
-    if (rc) return rc;
-    size_t o = 0;
-    for (size_t i = 0; i < k; ++i) {
-        const dgx_pack_view* v = views[i];
-        if (!v) continue;
-        const size_t nb = v->nblocks;
-        uint64_t* h_uoff = (uint64_t*)((char*)h_raw + o);
-        uint64_t acc = 0;
-        uint32_t max_num = 0;
-        for (size_t b = 0; b < nb; ++b) {
-            h_uoff[b] = acc;
-            const uint32_t num = v->num_uids[b];
-            acc += num;
-            max_num = std::max(max_num, num);
-            const uint64_t b0 = v->delta_off[b], b1 = v->delta_off[b + 1];
-            const uint64_t need = num > 1 ? 5ull * ((uint64_t)(num + 2) / 4) : 0;
-            if (b1 < b0 || b1 - b0 < need)
-                return fail(DGX_ERR_ARG, "malformed UidPack: block %zu has %lld delta bytes, NumUids %u needs >= %llu",
-                            b, (long long)(b1 - b0), num, (unsigned long long)need);
-        }
-        h_uoff[nb] = acc;
-        dgx_dev_pack& P = outs[i];
-        P.pk.nblocks = nb;
-        P.pk.base = (const u64*)dv[i].base;
-        P.pk.num = (const u32*)dv[i].num;
-        P.pk.delta_off = (const u64*)dv[i].doff;
-        P.pk.deltas = (const unsigned char*)dv[i].del;
-        P.pk.uid_off = (const u64*)((char*)d_raw + o);
-        P.pk.max_num = max_num;
-        P.pk.sysmem = 1;
-        P.d_mem = nullptr;
-        P.bytes = 0;
-        P.exact_len = acc;
-        P.block_size = v->block_size;
-        o += (nb + 1) * sizeof(uint64_t);
-        // the bytes still cross PCIe, as reads issued by the decode kernel
-        g_stats.h2d += nb * 20 + (nb + 1) * 8 + (size_t)v->delta_off[nb];
-    }
-    CK(cudaMemcpyAsync(d_raw, h_raw, uoff_total, cudaMemcpyHostToDevice, l->stream));
-    *done = true;
     return DGX_OK;
 }
 
@@ -1216,21 +1080,10 @@ static int packs_upload_run(dgx_lane* l, const dgx_pack_view* const* views, size
         const dgx_pack_view* v = views[i];
         if (!v) continue;
         const size_t nb = v->nblocks;
-        uint64_t* hu = (uint64_t*)((char*)h_uoff + uo);
-        uint64_t acc = 0;
+        uint64_t exact = 0;
         uint32_t max_num = 0;
-        for (size_t b = 0; b < nb; ++b) {
-            hu[b] = acc;
-            const uint32_t num = v->num_uids[b];
-            acc += num;
-            max_num = std::max(max_num, num);
-            const uint64_t b0 = v->delta_off[b], b1 = v->delta_off[b + 1];
-            const uint64_t need = num > 1 ? 5ull * ((uint64_t)(num + 2) / 4) : 0;
-            if (b1 < b0 || b1 - b0 < need)
-                return fail(DGX_ERR_ARG, "malformed UidPack: block %zu has %lld delta bytes, NumUids %u needs >= %llu",
-                            b, (long long)(b1 - b0), num, (unsigned long long)need);
-        }
-        hu[nb] = acc;
+        rc = pack_scan_blocks(v, (uint64_t*)((char*)h_uoff + uo), &exact, &max_num);
+        if (rc) return rc;
         char* d = (char*)d_img + ((const char*)v->base - start);
         dgx_dev_pack& P = outs[i];
         P.pk.nblocks = nb;
@@ -1240,10 +1093,9 @@ static int packs_upload_run(dgx_lane* l, const dgx_pack_view* const* views, size
         P.pk.deltas = (const unsigned char*)(d + image_meta_bytes(nb));
         P.pk.uid_off = (const u64*)((char*)d_uoff + uo);
         P.pk.max_num = max_num;
-        P.pk.sysmem = 0;
         P.d_mem = nullptr;
         P.bytes = view_image_bytes(v);
-        P.exact_len = acc;
+        P.exact_len = exact;
         P.block_size = v->block_size;
         uo += (nb + 1) * sizeof(uint64_t);
     }
@@ -1323,16 +1175,12 @@ static int decode_impl(dgx_lane* l, const DPack& pk, uint64_t seek, uint64_t* d_
     int rc = l->ws.alloc(sizeof(DSeek), &d_seek);
     if (rc) return rc;
     decode_seek_kernel<<<1, 32, 0, l->stream>>>(pk, seek, (DSeek*)d_seek, (u64*)d_out_len, out_cap, l->d_err);
-    CK(cudaGetLastError());
-    l->launches += 1;
-    g_stats.launches += 1;
+    if (int e = launched(l)) return e;
     if (pk.nblocks) {
         const uint64_t warps = (pk.nblocks + D_BPW - 1) / D_BPW;
         const uint64_t ctas = (warps + D_WARPS - 1) / D_WARPS;
         decode_kernel<<<(unsigned)ctas, D_NT, sizeof(DWarpSmem) * D_WARPS, l->stream>>>(pk, (const DSeek*)d_seek, (u64*)d_out, out_cap);
-        CK(cudaGetLastError());
-        l->launches += 1;
-        g_stats.launches += 1;
+        if (int e = launched(l)) return e;
     }
     return DGX_OK;
 }
@@ -1508,52 +1356,6 @@ extern "C" int dgx_merge_sorted(const uint64_t* const* lists, const size_t* lens
     return finish_to_host(l, (uint64_t*)d_len, (uint64_t*)d_out, total, out, out_cap, out_len);
 }
 
-extern "C" int dgx_intersect_batch(const uint64_t* a, const uint64_t* a_off, const uint64_t* b,
-                                   const uint64_t* b_off, size_t npairs, uint64_t* out, uint64_t* out_off,
-                                   size_t out_cap) {
-    if (npairs == 0) { if (out_off) out_off[0] = 0; return DGX_OK; }
-    LaneLease lease;
-    if (lease.rc) return lease.rc;
-    dgx_lane* l = lease.l;
-    g_stats.calls += 1;
-    const size_t na = a_off[npairs] - a_off[0], nbv = b_off[npairs] - b_off[0];
-    uint64_t *d_a, *d_b;
-    int rc = upload_list(l, a + a_off[0], na, &d_a);
-    if (rc) return rc;
-    rc = upload_list(l, b + b_off[0], nbv, &d_b);
-    if (rc) return rc;
-    std::vector<ListDesc> ld(2 * npairs);
-    std::vector<size_t> k_off(npairs + 1);
-    size_t cap = 0;
-    for (size_t i = 0; i < npairs; ++i) {
-        const size_t la = a_off[i + 1] - a_off[i], lb = b_off[i + 1] - b_off[i];
-        ld[2 * i] = {d_a + (a_off[i] - a_off[0]), la, nullptr};
-        ld[2 * i + 1] = {d_b + (b_off[i] - b_off[0]), lb, nullptr};
-        k_off[i] = 2 * i;
-        cap += std::min(la, lb);
-    }
-    k_off[npairs] = 2 * npairs;
-    void *d_out, *d_off;
-    rc = l->ws.alloc((cap + 2) * sizeof(uint64_t), &d_out);
-    if (rc) return rc;
-    rc = l->ws.alloc((npairs + 1) * sizeof(uint64_t), &d_off);
-    if (rc) return rc;
-    rc = filter_batch_impl(l, DGX_OP_INTERSECT, ld.data(), k_off.data(), npairs, (uint64_t*)d_out, cap, (uint64_t*)d_off);
-    if (rc) return rc;
-    CK(cudaMemcpyAsync(out_off, d_off, (npairs + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, l->stream));
-    rc = dgx_lane_sync(l);
-    if (rc) return rc;
-    const uint64_t n = out_off[npairs];
-    if (n > out_cap) return fail(DGX_ERR_CAP, "batch result (%llu) does not fit out_cap (%zu)", (unsigned long long)n, out_cap);
-    if (n) {
-        CK(cudaMemcpyAsync(out, d_out, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, l->stream));
-        CK(cudaStreamSynchronize(l->stream));
-    }
-    g_stats.d2h += (n + npairs + 1) * sizeof(uint64_t);
-    g_stats.uids_out += n;
-    return DGX_OK;
-}
-
 extern "C" int dgx_decode(const dgx_pack_view* p, uint64_t seek, uint64_t* out, size_t out_cap, size_t* out_len) {
     if (!p || p->nblocks == 0) {  // nil / empty pack decodes to the empty list (codec/codec.go:445-446)
         if (out_len) *out_len = 0;
@@ -1654,10 +1456,10 @@ static int icw_impl(dgx_lane* l, const dgx_dev_pack& pk, uint64_t after, const u
     // search the shorter side's elements in the longer side (the reference's linVsBinRatio idea, :49-59)
     if (m < nb) icw_ranges_by_v_kernel<<<(unsigned)((m + 255) / 256), 256, 0, l->stream>>>(P);
     else icw_ranges_by_block_kernel<<<(unsigned)((nb + 255) / 256), 256, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
+    if (int e = launched(l)) return e;
     const uint64_t warps = (nb + D_BPW - 1) / D_BPW;
     icw_probe_kernel<<<(unsigned)((warps + D_WARPS - 1) / D_WARPS), D_NT, sizeof(DWarpSmem) * D_WARPS, l->stream>>>(P);
-    CK(cudaGetLastError());
+    if (int e = launched(l)) return e;
     CompactParams C;
     C.v = (const u64*)d_v;
     C.keep = P.keep;
@@ -1669,9 +1471,7 @@ static int icw_impl(dgx_lane* l, const dgx_dev_pack& pk, uint64_t after, const u
     C.ticket = (u32*)((char*)d_raw + b_rng + b_keep + tiles * sizeof(u64));
     C.err = l->d_err;
     compact_kernel<<<(unsigned)tiles, CP_NT, 0, l->stream>>>(C);
-    CK(cudaGetLastError());
-    l->launches += 3;
-    g_stats.launches += 3;
+    if (int e = launched(l)) return e;
     g_stats.uids_in += pk.exact_len + m;
     return DGX_OK;
 }
@@ -1871,9 +1671,7 @@ static int decode_batch_impl(dgx_lane* l, const PackLease* pls, size_t k, uint64
     const u64 ctas = (warps + D_WARPS - 1) / D_WARPS;
     if (ctas > 0x7fffffffull) return fail(DGX_ERR_ARG, "packs too large for one decode launch");
     decode_batch_kernel<<<(unsigned)ctas, D_NT, sizeof(DWarpSmem) * D_WARPS, l->stream>>>((const DJob*)d_raw, nj, warps);
-    CK(cudaGetLastError());
-    l->launches += 1;
-    g_stats.launches += 1;
+    if (int e = launched(l)) return e;
     return DGX_OK;
 }
 
@@ -1900,9 +1698,7 @@ extern "C" int dgx_intersect_sorted_packed(const dgx_pack_ref* refs, size_t k, u
     }
     if (rc == DGX_OK) {
         std::vector<dgx_dev_pack> up(k);
-        bool mapped = false;
-        rc = packs_map_ws(l, oneshot.data(), k, up.data(), &mapped);  // pinned packs are decoded in place (zero-copy)
-        if (rc == DGX_OK && !mapped) rc = packs_upload_ws(l, oneshot.data(), k, up.data());
+        rc = packs_upload_ws(l, oneshot.data(), k, up.data());
         for (size_t i = 0; i < k && rc == DGX_OK; ++i)
             if (oneshot[i]) pls[i].pk = up[i];
     }
@@ -1984,9 +1780,7 @@ extern "C" int dgx_pack_seek(const dgx_pack_view* p, int kind, uint64_t uid, int
     S.out = (u64*)d_out;
     S.out_meta = (u64*)d_meta;
     pack_seek_kernel<<<1, 32, 0, l->stream>>>(S);
-    CK(cudaGetLastError());
-    l->launches += 1;
-    g_stats.launches += 1;
+    if (int e = launched(l)) return e;
     CK(cudaMemcpyAsync(l->h_word, d_meta, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, l->stream));
     CK(cudaMemcpyAsync(l->h_head, d_out, std::min(cap, kSpecHead) * sizeof(uint64_t), cudaMemcpyDeviceToHost, l->stream));
     rc = dgx_lane_sync(l);
@@ -2079,19 +1873,17 @@ static int encode_impl(dgx_lane* l, const uint64_t* d_u, size_t n, const uint64_
     // a list with more segments than seg_cap cannot be encoded into nblocks_cap blocks: the segment pass would
     // overrun its array, so it is bounded by the same capacity check (segments <= blocks)
     enc_segments_kernel<<<(unsigned)tiles_a, EN_NT, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
+    if (int e = launched(l)) return e;
     enc_segscan_kernel<<<1, 1024, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
+    if (int e = launched(l)) return e;
     const size_t warp_ctas = std::max<size_t>(1, (nblocks_cap * 32 + 255) / 256);
     enc_sizes_kernel<<<(unsigned)warp_ctas, 256, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
+    if (int e = launched(l)) return e;
     scan_u64_kernel<<<(unsigned)tiles_b, EN_NT, 0, l->stream>>>(P.blk_bytes, P.delta_off, P.counts + 1, nblocks_cap, status_b,
                                                                P.ticket + 1, P.counts + 2);
-    CK(cudaGetLastError());
+    if (int e = launched(l)) return e;
     enc_write_kernel<<<(unsigned)warp_ctas, 256, 0, l->stream>>>(P);
-    CK(cudaGetLastError());
-    l->launches += 5;
-    g_stats.launches += 5;
+    if (int e = launched(l)) return e;
     out->base = P.base; out->num = P.num; out->delta_off = P.delta_off; out->deltas = P.deltas; out->counts = P.counts;
     out->nblocks_cap = nblocks_cap; out->delta_cap = delta_cap;
     return DGX_OK;
@@ -2280,9 +2072,7 @@ extern "C" int dgx_index_of_batch(const uint64_t* u, size_t n, const uint64_t* u
     if (rc) return rc;
     const unsigned blocks = (unsigned)std::min<uint64_t>((m + 255) / 256, (uint64_t)g_num_sms * 16);
     index_of_kernel<<<blocks, 256, 0, l->stream>>>((const u64*)d_u, (u64)n, (const u64*)d_q, (u64)m, (long long*)d_idx);
-    CK(cudaGetLastError());
-    l->launches += 1;
-    g_stats.launches += 1;
+    if (int e = launched(l)) return e;
     g_stats.uids_in += n + m;
     CK(cudaMemcpyAsync(idx, d_idx, m * sizeof(int64_t), cudaMemcpyDeviceToHost, l->stream));
     g_stats.d2h += m * sizeof(int64_t);
@@ -2305,6 +2095,50 @@ static int batch_to_host(dgx_lane* l, const void* d_out, const void* d_off, size
     return DGX_OK;
 }
 
+// Intersects npairs pairs of uploaded lists and returns the results to the host.  List a of pair i is
+// d_a[a_off[i] - a_off[0], a_off[i + 1] - a_off[0]), list b is the same slice of d_b through b_off[i * b_step]:
+// b_step 1 gives every pair its own list b, b_step 0 gives all of them the one list [b_off[0], b_off[1]).
+static int intersect_pairs(dgx_lane* l, const uint64_t* d_a, const uint64_t* a_off, const uint64_t* d_b,
+                           const uint64_t* b_off, size_t b_step, size_t npairs, uint64_t* out, uint64_t* out_off,
+                           size_t out_cap) {
+    std::vector<ListDesc> ld(2 * npairs);
+    std::vector<size_t> k_off(npairs + 1);
+    size_t cap = 0;
+    for (size_t i = 0; i < npairs; ++i) {
+        const uint64_t* bo = b_off + i * b_step;
+        const size_t la = a_off[i + 1] - a_off[i], lb = bo[1] - bo[0];
+        ld[2 * i] = {d_a + (a_off[i] - a_off[0]), la, nullptr};
+        ld[2 * i + 1] = {d_b + (bo[0] - b_off[0]), lb, nullptr};
+        k_off[i] = 2 * i;
+        cap += std::min(la, lb);
+    }
+    k_off[npairs] = 2 * npairs;
+    void *d_out, *d_off;
+    int rc = l->ws.alloc((cap + 2) * sizeof(uint64_t), &d_out);
+    if (rc) return rc;
+    rc = l->ws.alloc((npairs + 1) * sizeof(uint64_t), &d_off);
+    if (rc) return rc;
+    rc = filter_batch_impl(l, DGX_OP_INTERSECT, ld.data(), k_off.data(), npairs, (uint64_t*)d_out, cap, (uint64_t*)d_off);
+    if (rc) return rc;
+    return batch_to_host(l, d_out, d_off, npairs, out, out_off, out_cap);
+}
+
+extern "C" int dgx_intersect_batch(const uint64_t* a, const uint64_t* a_off, const uint64_t* b,
+                                   const uint64_t* b_off, size_t npairs, uint64_t* out, uint64_t* out_off,
+                                   size_t out_cap) {
+    if (npairs == 0) { if (out_off) out_off[0] = 0; return DGX_OK; }
+    LaneLease lease;
+    if (lease.rc) return lease.rc;
+    dgx_lane* l = lease.l;
+    g_stats.calls += 1;
+    uint64_t *d_a, *d_b;
+    int rc = upload_list(l, a + a_off[0], a_off[npairs] - a_off[0], &d_a);
+    if (rc) return rc;
+    rc = upload_list(l, b + b_off[0], b_off[npairs] - b_off[0], &d_b);
+    if (rc) return rc;
+    return intersect_pairs(l, d_a, a_off, d_b, b_off, 1, npairs, out, out_off, out_cap);
+}
+
 extern "C" int dgx_intersect_batch_shared(const uint64_t* a, const uint64_t* a_off, size_t npairs, const uint64_t* b,
                                           size_t m, uint64_t* out, uint64_t* out_off, size_t out_cap) {
     if (npairs == 0) { if (out_off) out_off[0] = 0; return DGX_OK; }
@@ -2313,31 +2147,13 @@ extern "C" int dgx_intersect_batch_shared(const uint64_t* a, const uint64_t* a_o
     if (lease.rc) return lease.rc;
     dgx_lane* l = lease.l;
     g_stats.calls += 1;
-    const size_t na = a_off[npairs] - a_off[0];
     uint64_t *d_a, *d_b;
-    int rc = upload_list(l, a + a_off[0], na, &d_a);
+    int rc = upload_list(l, a + a_off[0], a_off[npairs] - a_off[0], &d_a);
     if (rc) return rc;
     rc = upload_list(l, b, m, &d_b);  // the shared list crosses PCIe once
     if (rc) return rc;
-    std::vector<ListDesc> ld(2 * npairs);
-    std::vector<size_t> k_off(npairs + 1);
-    size_t cap = 0;
-    for (size_t i = 0; i < npairs; ++i) {
-        const size_t la = a_off[i + 1] - a_off[i];
-        ld[2 * i] = {d_a + (a_off[i] - a_off[0]), la, nullptr};
-        ld[2 * i + 1] = {d_b, m, nullptr};
-        k_off[i] = 2 * i;
-        cap += std::min(la, m);
-    }
-    k_off[npairs] = 2 * npairs;
-    void *d_out, *d_off;
-    rc = l->ws.alloc((cap + 2) * sizeof(uint64_t), &d_out);
-    if (rc) return rc;
-    rc = l->ws.alloc((npairs + 1) * sizeof(uint64_t), &d_off);
-    if (rc) return rc;
-    rc = filter_batch_impl(l, DGX_OP_INTERSECT, ld.data(), k_off.data(), npairs, (uint64_t*)d_out, cap, (uint64_t*)d_off);
-    if (rc) return rc;
-    return batch_to_host(l, d_out, d_off, npairs, out, out_off, out_cap);
+    const uint64_t b_off[2] = {0, m};
+    return intersect_pairs(l, d_a, a_off, d_b, b_off, 0, npairs, out, out_off, out_cap);
 }
 
 // ---------------------------------------------------------------------------

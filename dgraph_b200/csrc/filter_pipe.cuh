@@ -57,9 +57,6 @@ constexpr int P_OS = DGX_P_OS;           // output slots in flight (6 vs 4: 2-li
 #ifndef DGX_P_ST
 #define DGX_P_ST 2
 #endif
-#ifndef DGX_PLAN_4ARY
-#define DGX_PLAN_4ARY 0   // 1: 4-ary plan searches (half the dependent latencies, 1.5x the probes) -- measured 2.4 % SLOWER on C2
-#endif
 #ifndef DGX_P_PAIR2
 #define DGX_P_PAIR2 1   // two-row warps search two lists per iteration (four chains) once past the first list
 #endif
@@ -131,30 +128,6 @@ __global__ void __launch_bounds__(256) filter_plan_kernel(const FTask* __restric
         const FList Lj = lists[T.list_first + j];
         const u64* __restrict__ B = Lj.ptr;
         u64 l0 = 0, h0 = flist_len(Lj), l1 = 0, h1 = h0;
-#if DGX_PLAN_4ARY
-        // Both searches advance in lock step and 4-ary: three probes per search and level are in flight together, so
-        // the dependent chain is log4(n) memory latencies instead of log2(n) -- the kernel is a latency chain, not a
-        // bandwidth load (the extra probes touch ~1.5x the sectors of a binary search, a few MB per launch)
-        while (h0 - l0 > 3 || h1 - l1 > 3) {
-            const bool a = h0 - l0 > 3, c = h1 - l1 > 3;
-            const u64 q0 = (h0 - l0) >> 2, q1 = (h1 - l1) >> 2;
-            u64 a1 = 0, a2 = 0, a3 = 0, c1 = 0, c2 = 0, c3 = 0;
-            if (a) { a1 = ld_probe(B + l0 + q0); a2 = ld_probe(B + l0 + 2 * q0); a3 = ld_probe(B + l0 + 3 * q0); }
-            if (c) { c1 = ld_probe(B + l1 + q1); c2 = ld_probe(B + l1 + 2 * q1); c3 = ld_probe(B + l1 + 3 * q1); }
-            if (a) {
-                if (a3 < tlo) l0 = l0 + 3 * q0 + 1;
-                else if (a2 < tlo) { h0 = l0 + 3 * q0; l0 = l0 + 2 * q0 + 1; }
-                else if (a1 < tlo) { h0 = l0 + 2 * q0; l0 = l0 + q0 + 1; }
-                else h0 = l0 + q0;
-            }
-            if (c) {
-                if (c3 <= thi) l1 = l1 + 3 * q1 + 1;
-                else if (c2 <= thi) { h1 = l1 + 3 * q1; l1 = l1 + 2 * q1 + 1; }
-                else if (c1 <= thi) { h1 = l1 + 2 * q1; l1 = l1 + q1 + 1; }
-                else h1 = l1 + q1;
-            }
-        }
-#endif
         while (l0 < h0 || l1 < h1) {
             const u64 m0 = l0 + ((h0 - l0) >> 1), m1 = l1 + ((h1 - l1) >> 1);
             const bool a = l0 < h0, c = l1 < h1;

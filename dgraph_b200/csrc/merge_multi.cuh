@@ -1,4 +1,4 @@
-// merge_multi.cuh -- single-pass multiway MergeSorted (k <= 64 runs) for sm_100a.
+// merge_multi.cuh -- single-pass multiway MergeSorted (k <= 64 runs) for sm_100a: shared pieces.
 //
 // algo.MergeSorted (algo/uidlist.go:448-542) pops a k-way heap and drops values equal
 // to the last one written: a sorted union with global de-duplication.  A pairwise
@@ -8,18 +8,17 @@
 //   (merge tree)     the k sample runs are themselves sorted, so the existing pairwise
 //                    merge tree (merge_kernel, with de-duplication) turns them into the
 //                    sorted distinct splitters; splitters b-1 .. b bound tile b.
-//   mplan_kernel     one thread per (boundary, run): lower_bound of the splitter in the run
-//   mmerge_kernel    one CTA per tile: the k slices of the tile's value range are merged in
-//                    shared memory by log2(k) rounds of pairwise merge-path merges, values
-//                    equal to their predecessor are dropped, the result goes to a scratch
-//                    buffer at the tile's INPUT offset (output <= input, so regions never
-//                    overlap) and the tile's count is recorded.  A tile larger than the
-//                    shared-memory chunk is processed in rounds: every run contributes a
-//                    quota, only values <= the smallest "last loaded value of a run that has
-//                    more" are final in that round (classic block-wise k-way merge), so no
-//                    distribution of the input can overflow shared memory.
+//   mplan2_kernel    position of every splitter in every run (merge_tile32.cuh)
+//   mmerge3_kernel   one CTA per tile merges the tile's slices of the k runs, drops repeats
+//                    and writes the result to a scratch buffer at the tile's INPUT offset
+//                    (output <= input, so regions never overlap) (merge_tile32.cuh)
 //   mscan_kernel     exclusive scan of the tile counts (one CTA)
 //   mcompact_kernel  moves every tile's output to its final, compact position.
+// This file holds the 64-bit tile engine (mm_levels_tile), which mmerge3_kernel runs for
+// tiles whose value span does not fit 32 bits.  A tile larger than the shared-memory chunk
+// is processed in rounds: every run contributes a quota, only values <= the smallest "last
+// loaded value of a run that has more" are final in that round (classic block-wise k-way
+// merge), so no distribution of the input can overflow shared memory.
 #pragma once
 
 #include "common.cuh"
@@ -47,7 +46,7 @@ struct MMParams {
     u64* splitters;         // <= nsamp
     const u64* nsplit;      // device word: number of distinct sample values
     u32 stride;             // every stride-th distinct sample is a splitter (evens out tile sizes)
-    u64* bounds;            // (nsamp + 2) * k: boundary b, run j -> position in run j
+    u64* bounds;            // k * nbs, run-major: bounds[j * nbs + b] = position of boundary b in run j
     u64* tile_in;           // nsamp + 1: input offset of every tile (= scratch offset)
     u32* tile_cnt;          // nsamp + 1: values the tile produced
     u64* tile_out;          // nsamp + 2: exclusive scan of tile_cnt
@@ -56,12 +55,8 @@ struct MMParams {
     u64 out_cap;
     u64* out_len;
     int* err;
-    // merge_tile32.cuh
-    u32 nbs;                // boundaries per run in the run-major bounds table (bounds[j * nbs + b])
-    u64* status;            // look-back words, one per tile, zeroed
-    u32* ticket;            // zeroed
-    u32 ahead;              // merge_tile32.cuh: prefetch the tile this many tiles on into L2 (0 = off)
-    u32 lag;                // merge_tile32.cuh: a CTA moves the tile `lag` tiles before its own to the output (0 = scan + compact kernels)
+    u32 nbs;                // boundaries per run in the bounds table
+    u32 ahead;              // prefetch the tile this many tiles on into L2 (0 = off)
     u64* tile_lo;           // nsamp + 2: base of a tile's 32-bit scratch keys
 };
 
@@ -81,22 +76,6 @@ __global__ void __launch_bounds__(256) msample_kernel(const MMParams P) {
     u64 v = kU64Max;  // an empty (fully de-duplicated) run contributes "+inf" samples
     if (n > 0) v = ld_probe(p + (u64)(((unsigned __int128)(r + 1) * n) / (s + 1)));
     P.samples[i] = v;
-}
-
-// ---- boundaries: position of every splitter in every run ----------------------------------
-__global__ void __launch_bounds__(256) mplan_kernel(const MMParams P) {
-    const u32 ns = (u32)(*P.nsplit / P.stride);
-    const u64 idx = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    const u64 nb = (u64)ns + 2;  // boundaries 0 .. ns+1
-    if (idx >= nb * P.k) return;
-    const u32 b = (u32)(idx / P.k), j = (u32)(idx % P.k);
-    const u64* p; u64 n;
-    mref_resolve(P.runs[j], p, n);
-    u64 pos;
-    if (b == 0) pos = 0;
-    else if (b == ns + 1) pos = n;
-    else pos = lower_bound_g(p, n, P.splitters[(u64)b * P.stride - 1]);
-    P.bounds[idx] = pos;
 }
 
 // ---- the merge -----------------------------------------------------------------------------
@@ -142,7 +121,7 @@ __device__ __forceinline__ void mm_merge_level(const u64* src, u64* dst, const i
 // most MM_C values (two ping-pong buffers of MM_CP values in s_mm), values equal to their predecessor are dropped and
 // the rest is appended to dst.  Called by all MM_NT threads of the CTA; returns the number of values written.
 __device__ __noinline__ u32 mm_levels_tile(u64* s_mm, const u64* const* s_ptr, u64* s_cur, const u64* s_end, int k,
-                                           u64* dst, bool have_last, u64 last) {
+                                           u64* dst) {
     u64* s_x = s_mm;
     u64* s_y = s_mm + MM_CP;
     __shared__ int s_off[2][MM_K + 2];
@@ -152,6 +131,10 @@ __device__ __noinline__ u32 mm_levels_tile(u64* s_mm, const u64* const* s_ptr, u
     __shared__ u32 s_scan[MM_NT / 32 + 1];
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     u32 produced = 0;
+    // A value equal to a round's bound can have more copies waiting in runs that had loaded only part of them, so the
+    // last value written is remembered across rounds.
+    bool have_last = false;
+    u64 last = 0;
 
     for (;;) {
         // ---- how much of every run enters this round -------------------------------------------
@@ -300,55 +283,6 @@ __device__ __noinline__ u32 mm_levels_tile(u64* s_mm, const u64* const* s_ptr, u
         if (fits) break;
     }
     return produced;
-}
-
-__global__ void __launch_bounds__(MM_NT, 3) mmerge_kernel(const MMParams P) {
-    extern __shared__ __align__(16) u64 s_mm[];  // two ping-pong buffers of MM_C values
-    __shared__ u64 s_cur[MM_K], s_end[MM_K];
-    __shared__ const u64* s_ptr[MM_K];
-    __shared__ u64 s_red[8];
-
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const u32 b = blockIdx.x;
-    const u32 ns = (u32)(*P.nsplit / P.stride);
-    if (b > ns) return;
-    const int k = (int)P.k;
-
-    // ---- the tile's slice of every run, its input offset and its predecessor value ------------
-    u64 my_c = 0;
-    u64 my_pred = 0;
-    bool my_has = false;
-    if (tid < k) {
-        const u64* p; u64 n;
-        mref_resolve(P.runs[tid], p, n);
-        const u64 c = P.bounds[(u64)b * k + tid], e = P.bounds[(u64)(b + 1) * k + tid];
-        s_ptr[tid] = p; s_cur[tid] = c; s_end[tid] = e;
-        my_c = c;
-        if (c > 0) { my_pred = ld_probe(p + c - 1); my_has = true; }
-    }
-    // block reductions over the first 64 threads (two warps): sum of starts, max predecessor
-    {
-        u64 sum = my_c, mx = my_has ? my_pred : 0;
-        u32 any = my_has ? 1u : 0u;
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            sum += __shfl_xor_sync(0xffffffffu, sum, d);
-            const u64 o = __shfl_xor_sync(0xffffffffu, mx, d);
-            mx = o > mx ? o : mx;
-            any |= __shfl_xor_sync(0xffffffffu, any, d);
-        }
-        if (lane == 0 && wid < 2) { s_red[wid] = sum; s_red[2 + wid] = mx; s_red[4 + wid] = any; }
-    }
-    __syncthreads();
-    const u64 inbase = s_red[0] + s_red[1];
-    const bool have_last = (s_red[4] | s_red[5]) != 0;
-    const u64 last = s_red[2] > s_red[3] ? s_red[2] : s_red[3];
-    __syncthreads();
-    const u32 produced = mm_levels_tile(s_mm, s_ptr, s_cur, s_end, k, P.scratch + inbase, have_last, last);
-    if (tid == 0) {
-        P.tile_in[b] = inbase;
-        P.tile_cnt[b] = produced | 0x80000000u;  // scratch holds u64 values (mcompact_kernel)
-    }
 }
 
 // ---- scan of the tile counts (one CTA) --------------------------------------------------------

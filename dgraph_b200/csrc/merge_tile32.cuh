@@ -1,10 +1,10 @@
-// merge_tile32.cuh -- the tile engine of the single-pass multiway MergeSorted, second version.
+// merge_tile32.cuh -- the bounds and tile kernels of the single-pass multiway MergeSorted.
 //
-// Same decomposition as merge_multi.cuh (samples -> distinct splitters -> per-(boundary, run) bounds -> one CTA per
-// tile -> scan of the tile counts -> compaction), with two changes:
+// The pipeline (samples -> distinct splitters -> per-(boundary, run) bounds -> one CTA per tile -> scan of the tile
+// counts -> compaction) is described in merge_multi.cuh.  The two kernels here:
 //   mplan2_kernel   bounds, run-major (threads of a warp search neighbouring splitters in the SAME run, so their
 //                   probes share sectors), each search confined to the gap between two samples of the run (the
-//                   samples are already in HBM/L2: 9 steps instead of 24).
+//                   samples are already in HBM/L2: 9 steps instead of 24 over the whole run).
 //   mmerge3_kernel  all values of a tile lie in [lo, hi]; when hi - lo fits 32 bits (any realistic uid distribution)
 //                   the k slices are loaded as 32-bit offsets from lo and the six levels of pairwise merge-path merges
 //                   run on u32 keys: one-instruction compares and selects, half the shared-memory bytes (so a
@@ -347,82 +347,19 @@ __device__ __noinline__ u32 t32_tile(u32* s_k, const u64* const* s_ptr, u64* s_c
     return produced;
 }
 
-// ---- lagged compaction (optional: DGX_MERGE_LAG > 0; default is mscan_kernel + mcompact_kernel) --------------------
-// A tile's place in the output is the sum of the counts of the tiles before it, known only when they are all done.
-// Waiting for it at the end of a tile retires the CTAs in order (measured: half the kernel's time spent waiting behind
-// the slowest tile).  Here a tile writes its keys to scratch, publishes its count, and the CTA that starts P.lag tiles
-// LATER -- when the tile and its predecessors have long finished -- resolves the offset with a decoupled look-back that
-// finds everything already published, and moves the values to their final position before it begins its own tile;
-// mtail_kernel moves the last P.lag tiles.  Bit-exact, no waiting at lag >= 6 x SMs, but measured no faster than the
-// two extra kernels (C5: 1.69 vs 1.655 ms): the merge kernel is bound by its phases' latencies, not by issue slots, so
-// the copy phase costs what the compaction kernel costs.
 constexpr u32 kTileWide = 0x80000000u;  // tile_cnt flag: the tile's scratch holds u64 values, not u32 offsets from tile_lo
-
-__device__ __forceinline__ u64 t32_ldcg64(const u64* p) {
-    u64 v;
-    asm volatile("ld.global.cg.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ u32 t32_ldcg32(const u32* p) {
-    u32 v;
-    asm volatile("ld.global.cg.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-
-// One warp: output offset of tile t (its count must be, or is about to be, published in P.status[t]).
-// Returns the exclusive prefix; *agg gets the tile's count.
-__device__ __forceinline__ u64 t32_tile_offset(const MMParams& P, u32 t, int lane, u64* agg) {
-    u64 w = 0;
-    if (lane == 0) {
-        while (((w = ld_relaxed(P.status + t)) >> 62) == 0) __nanosleep(200);
-    }
-    w = __shfl_sync(0xffffffffu, w, 0);
-    *agg = w & kValMask;
-    const u64 base = lookback_exclusive<true, 100>(P.status, t, *agg, lane);
-    __threadfence();  // what the tile wrote before publishing its count is visible to the loads that follow
-    return base;
-}
-
-// All threads of the CTA: move tile t's values from scratch to out[base ..).
-template <int NT>
-__device__ __forceinline__ void t32_copy_tile(const MMParams& P, u32 t, u64 base, int tid) {
-    const u64 inb = t32_ldcg64(P.tile_in + t);
-    const u64 lo = t32_ldcg64(P.tile_lo + t);
-    const u32 c = t32_ldcg32(P.tile_cnt + t);
-    const u32 cnt = c & ~kTileWide;
-    if (c & kTileWide) {
-        const u64* src = P.scratch + inb;
-        for (u32 i = tid; i < cnt; i += NT)
-            if (base + i < P.out_cap) st_stream(P.out + base + i, t32_ldcg64(src + i));
-    } else {
-        const u32* src = (const u32*)(P.scratch + inb);
-        for (u32 i = tid; i < cnt; i += NT)
-            if (base + i < P.out_cap) st_stream(P.out + base + i, lo + t32_ldcg32(src + i));
-    }
-}
 
 __global__ void __launch_bounds__(T_NT, 3) mmerge3_kernel(const MMParams P) {
     extern __shared__ __align__(16) unsigned char s_raw[];
     __shared__ u64 s_cur[MM_K], s_end[MM_K];
     __shared__ const u64* s_ptr[MM_K];
     __shared__ u64 s_r[2][4];
-    __shared__ u64 s_cbase;
-    __shared__ u32 s_tile;
 
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    // tiles are numbered in the order their CTAs start, so every tile before a running one has started (look-back)
-    if (tid == 0) s_tile = P.lag ? atomicAdd(P.ticket, 1u) : blockIdx.x;
-    __syncthreads();
-    const u32 b = s_tile;
+    const u32 b = blockIdx.x;
     const u32 ns = (u32)(*P.nsplit / P.stride);
     if (b > ns) return;
     const int k = (int)P.k;
-    const bool docopy = P.lag != 0 && b >= P.lag;
-    if (docopy && wid == 2) {  // warps 0 and 1 read the tile's bounds meanwhile
-        u64 agg;
-        const u64 base = t32_tile_offset(P, b - P.lag, lane, &agg);
-        if (lane == 0) s_cbase = base;
-    }
 
     // ---- the tile's slice of every run; input offset, size, smallest and largest value ---------------------
     // An interior tile holds the values in [S(b), S(b+1)) (S(b) = splitter of boundary b), which bounds its span without
@@ -474,7 +411,6 @@ __global__ void __launch_bounds__(T_NT, 3) mmerge3_kernel(const MMParams P) {
         const u64* q = s_ptr[tid];
         for (u64 i = c2 & ~(u64)15; i < e2; i += 16) asm volatile("prefetch.global.L2 [%0];" ::"l"(q + i));
     }
-    if (docopy) t32_copy_tile<T_NT>(P, b - P.lag, s_cbase, tid);
 
     // Equal values always fall into the same tile (every run is cut at lower_bound of the same splitter), so a tile
     // never has to look at its predecessor's last value.
@@ -482,40 +418,13 @@ __global__ void __launch_bounds__(T_NT, 3) mmerge3_kernel(const MMParams P) {
     const bool wide = hi - lo >= (u64)T_INF;
     if (total != 0) {
         if (!wide) produced = t32_tile((u32*)s_raw, s_ptr, s_cur, s_end, k, (u32*)(P.scratch + inbase), lo);
-        else produced = mm_levels_tile((u64*)s_raw, s_ptr, s_cur, s_end, k, P.scratch + inbase, false, 0);
+        else produced = mm_levels_tile((u64*)s_raw, s_ptr, s_cur, s_end, k, P.scratch + inbase);
     }
-    __syncthreads();  // every thread's scratch writes precede the fence below
     if (tid == 0) {
         P.tile_in[b] = inbase;
         P.tile_lo[b] = lo;
         P.tile_cnt[b] = produced | (wide ? kTileWide : 0u);
-        if (P.lag) {
-            __threadfence();
-            st_relaxed(P.status + b, kFlagAgg | (u64)produced);
-        }
     }
-}
-
-// The tiles no later CTA moves: tile ns - i for CTA i < min(lag, ns + 1).  The CTA of tile ns also reports the length.
-__global__ void __launch_bounds__(T_NT) mtail_kernel(const MMParams P) {
-    __shared__ u64 s_cbase;
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const u32 ns = (u32)(*P.nsplit / P.stride);
-    if (blockIdx.x > ns) return;
-    const u32 t = ns - blockIdx.x;
-    if (wid == 0) {
-        u64 agg;
-        const u64 base = t32_tile_offset(P, t, lane, &agg);
-        if (lane == 0) {
-            s_cbase = base;
-            if (t == ns) {
-                *P.out_len = base + agg;
-                if (base + agg > P.out_cap) atomicExch(P.err, 1);
-            }
-        }
-    }
-    __syncthreads();
-    t32_copy_tile<T_NT>(P, t, s_cbase, tid);
 }
 
 }  // namespace dgx

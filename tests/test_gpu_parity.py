@@ -381,22 +381,21 @@ def test_properties_at_scale(dgx):
     eq(m2.Uids, np.union1d(a, b), "union")
 
 
-@pytest.mark.parametrize("knobs", [{}, {"DGX_MERGE_STRIDE": "16"}, {"DGX_MERGE_LAG": "3"}, {"DGX_MERGE_LAG": "700"},
-                                   {"DGX_MERGE": "levels"}],
-                         ids=["default", "stride16", "lag3", "lag700", "levels"])
+@pytest.mark.parametrize("knobs", [{}, {"DGX_MERGE_STRIDE": "16"}, {"DGX_MERGE": "tree"}],
+                         ids=["default", "stride16", "tree"])
 def test_merge_multiway_forced(orc, knobs):
     """The multiway MergeSorted path with its size threshold removed (DGX_MERGE_MULTI_MIN=0), in a
     subprocess because libdgx reads its knobs once: known answers, random k, adversarial shapes that
     force the block-wise rounds (identical lists, one dense cluster, long duplicate runs).  Variants: tiles so large
-    that most need several rounds (stride 16), compaction inside the merge kernel at a lag smaller and larger than
-    the number of resident CTAs, and the round-1 pipeline (64-bit tile keys)."""
+    that most need several rounds (stride 16), and the pairwise tree forced for every k.  The launch count of a small
+    k = 9 merge shows which path ran: the tree takes ceil(log2 9) = 4 launches, the multiway path more."""
     import subprocess
     code = r'''
 import os, sys
 import numpy as np
 sys.path.insert(0, os.getcwd()); sys.path.insert(0, os.path.join(os.getcwd(), "tests"))
 import gen
-from dgraph_b200 import algo, pb
+from dgraph_b200 import _lib, algo, pb
 from oracle import pyoracle as orc
 from test_oracle_algo import MERGE_CASES
 def L(x): return pb.List(np.asarray(x, dtype=np.uint64))
@@ -404,6 +403,13 @@ def chk(lists, what):
     got = algo.MergeSorted([L(l) for l in lists]).Uids
     want = orc.merge_sorted(lists)
     assert got.size == want.size and np.array_equal(got, want), (what, got.size, want.size)
+before = _lib.stats()["kernel_launches"]
+chk([np.arange(j, 9000, 9, dtype=np.uint64) for j in range(9)], "k=9, 9000 values")
+launches = _lib.stats()["kernel_launches"] - before
+if os.environ.get("DGX_MERGE") == "tree":
+    assert launches == 4, ("forced tree", launches)
+else:
+    assert launches > 4, ("multiway threshold not lifted", launches)
 for lists, want in MERGE_CASES:
     got = algo.MergeSorted([L(l) for l in lists])
     assert got.tolist() == want, (lists, got.tolist())

@@ -15,7 +15,7 @@ timeout 400 ncu --set full --clock-control none --import-source on -k regex:filt
     python bench.py --steps 3 --warmup 3 --no-e2e --no-ops --no-dense > $o/${tag}_ncu_pipe.log 2>&1
 timeout 300 ncu --set full --clock-control none --import-source on -k regex:mmerge3_kernel -s 1 -c 1 -f -o $o/${tag}_mmerge \
     python tools/prof_merge.py 100000000 > $o/${tag}_ncu_merge.log 2>&1
-timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -k 'regex:^(msample|mplan2?|mmerge3?|mscan|mcompact|mtail|merge)_kernel' -c 60 --csv --log-file $o/${tag}_merge_launches.csv \
+timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -k 'regex:^(msample|mplan2|mmerge3|mscan|mcompact|merge)_kernel' -c 60 --csv --log-file $o/${tag}_merge_launches.csv \
     python tools/prof_merge.py 100000000 > $o/${tag}_ncu_merge2.log 2>&1
 timeout 300 ncu --set full --clock-control none --import-source on -k regex:decode_kernel -s 1 -c 1 -f -o $o/${tag}_decode \
     python tools/prof_decode.py > $o/${tag}_ncu_decode.log 2>&1
